@@ -24,6 +24,7 @@ import time
 import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -87,7 +88,36 @@ def parse_args():
                          "65544-byte IDAT chunks: chunk CRC-32 and IDAT gather on the device)")
     ap.add_argument("--e2e-sweep", default="", help="experiment: comma list of LANESxCHUNKS_PER_LANE to time the host leg with")
     ap.add_argument("--cpu-images", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one decoded (rank 0's batch) to DIR/*.npy: "
+                         "per-image status, checksum and produced bytes, and a seeded sample of the pixel bytes")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "decode"):
+        ap.error("--dump-outputs writes the outputs of the GPU decode path (--impl ours --mode decode)")
+    return args
+
+
+DUMP_SAMPLES = 1 << 22  # pixel bytes kept by --dump-outputs: 16 MiB of float32 values + 32 MiB of float64 offsets
+
+
+def dump_outputs(out_dir, d_pixels, descs, B):
+    """What a caller of pngb200_decode_batch receives, as float arrays: the per-image result words in full and
+    the decoded pixel bytes at DUMP_SAMPLES offsets drawn from a fixed seed (the same ones for the same
+    workload and batch, so that two builds can be compared output for output)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = d_pixels.numel()
+    if total <= DUMP_SAMPLES:
+        index = np.arange(total, dtype=np.int64)
+    else:
+        index = np.unique(np.random.default_rng(0).integers(0, total, DUMP_SAMPLES, dtype=np.int64))
+    sample = d_pixels.view(-1)[torch.from_numpy(index).to(d_pixels.device)]
+    arrays = {"status": [descs[i].status for i in range(B)], "checksum": [descs[i].checksum for i in range(B)],
+              "produced": [descs[i].produced for i in range(B)], "pixels_sample": sample.float().cpu().numpy(),
+              "pixels_sample_offset": index}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"),
+                np.asarray(a, dtype=np.float32 if name == "pixels_sample" else np.float64))
 
 
 # ------------------------------------------------------------------ corpus
@@ -334,6 +364,8 @@ def main():
         barrier()
     ms = ev0.elapsed_time(ev1)
     launches = ctx.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_pixels, descs, B)
     stats = ctx.inflate_counters(B)
     engine_used = ctx.last_inflate_engine()
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")

@@ -10,7 +10,6 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):

@@ -1,6 +1,8 @@
-"""Regenerates tests/golden/ from the reference checkout (run in the build container, where
-/root/reference exists).  The GPU box has no /root/reference, so everything the tests need from
-the reference's fixtures is committed here:
+"""Regenerates tests/golden/ from a checkout of the reference (swift-png), given as the only argument:
+
+    python tests/golden/make_golden.py PATH-TO-SWIFT-PNG
+
+The tests never read the reference itself, so everything they need from its fixtures is committed here:
 
   pngsuite/*.png            the reference's PngSuite inputs (Sources/PNGIntegrationTests/Inputs/Common)
   invalid/*.png             its malformed inputs              (.../Inputs/Invalid)
@@ -12,6 +14,8 @@ the reference's fixtures is committed here:
   encode/*.png (+ .json)    a subset of the reference encoder's committed level-9 outputs
                             (Tests/Outputs) with the matching Tests/Baselines inputs, and
                             sha256 digests of the concatenated IDAT payload for all 28
+  outputs/*.png             more of those level-9 outputs, without their inputs: the smallest one of
+                            each 8-bit pixel layout encode/ does not hold (all 28 are 4.4 MB)
 """
 import hashlib
 import json
@@ -21,7 +25,7 @@ import struct
 import sys
 import zlib
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+REF = sys.argv[1]
 HERE = os.path.dirname(os.path.abspath(__file__))
 IT = os.path.join(REF, "Sources", "PNGIntegrationTests")
 
@@ -71,6 +75,8 @@ def main():
     os.makedirs(os.path.join(HERE, "encode"), exist_ok=True)
     keep = {"rgba8-color-photographic.png", "v8-monochrome-nonphotographic.png",
             "rgb16-color-nonphotographic.png", "indexed8-color-photographic.png"}
+    sampled = {"va8-monochrome-nonphotographic.png", "rgb8-monochrome-nonphotographic.png"}
+    os.makedirs(os.path.join(HERE, "outputs"), exist_ok=True)
     outs = os.path.join(REF, "Tests", "Outputs")
     for f in sorted(os.listdir(outs)):
         if not f.endswith(".png"):
@@ -86,6 +92,8 @@ def main():
             shutil.copyfile(os.path.join(outs, f), os.path.join(HERE, "encode", "out-" + f))
             shutil.copyfile(os.path.join(REF, "Tests", "Baselines", f),
                             os.path.join(HERE, "encode", "in-" + f))
+        if f in sampled:
+            shutil.copyfile(os.path.join(outs, f), os.path.join(HERE, "outputs", f))
     json.dump(enc, open(os.path.join(HERE, "encode.json"), "w"), indent=0, sort_keys=True)
 
 
